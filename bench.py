@@ -33,6 +33,9 @@ cpu_baseline / --impl reference: the reference's OWN classes on the host
 Launch: python bench.py [--gpus N --steps K --warmup W]; for N > 1 under
 torch.distributed.run (one rank per GPU, NCCL only for the timing barrier and
 max-reduction: the replay shards never exchange data -> "scaling": "weak").
+--dump-outputs DIR writes the minibatch the last timed exact pass returned
+(rank 0) as DIR/<name>.npy; the inputs are seeded, so two builds run with the
+same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -63,6 +66,8 @@ ALGO_BYTES_TREE = 1684
 ALGO_BYTES_PATH = ALGO_BYTES_GATHER + ALGO_BYTES_TREE
 # uint8 batches out (x/255 folded into conv1): 7 frames read + 2 x 4 frames written = 107.6 KB
 ALGO_BYTES_PATH_U8 = 7 * FRAME_BYTES + 2 * STACK * FRAME_BYTES + 32 + ALGO_BYTES_TREE
+# --dump-outputs: rows of state / next_state written (2 x 64 x 113 KB = 14.5 MB)
+DUMP_ROWS = 64
 
 
 def parse():
@@ -81,7 +86,13 @@ def parse():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-rainbow-graph", action="store_true",
                     help="run the Rainbow learn step eagerly instead of as one CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline pass returned in its last timed step to "
+                         "DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 # ---------------------------------------------------------------------------
@@ -421,6 +432,8 @@ def main():
         print(json.dumps(line))
         return
 
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)  # fail before the run, not after it
     import torch
     import torch.distributed as dist
 
@@ -564,10 +577,26 @@ def main():
                                          "ascent_wait": ph[20] / B, "ascent_work": ph[21] / B}}
                                         if ph[5] else {})}
 
+    def last_step_outputs():
+        """The minibatch the last exact pass handed its caller, as float32 / float64 arrays
+        (indices and actions exactly); state / next_state as DUMP_ROWS rows drawn with a
+        fixed seed (state_rows), which keeps the dump far below 64 MB."""
+        rows = np.sort(np.random.RandomState(0).choice(B, min(B, DUMP_ROWS), replace=False))
+        sel = torch.from_numpy(rows).to(dev)
+        out = {"index": o_index.double(), "weight": o_weight, "action": o_action.double(),
+               "reward": o_reward, "terminal": o_term, "discount": o_disc,
+               "state": o_state[sel].view(-1, STACK, *FRAME),
+               "next_state": o_next[sel].view(-1, STACK, *FRAME)}
+        out = {k: v.cpu().numpy() for k, v in out.items()}
+        out["state_rows"] = rows.astype(np.float64)
+        return out
+
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()  # samples SM clock / throttle reasons through all timed regions
     ms_value, phases_exact = fused_loop(_lib.SAMPLE_EXACT)
+    # taken now: the loops below reuse the output tensors
+    dumped = last_step_outputs() if args.dump_outputs and rank == 0 else None
     scout = store.info()["scout_hits"]
     ms_par, phases_par = fused_loop(_lib.SAMPLE_PARALLEL)
     # the same pass emitting uint8 batches (x/255 folded into the first conv layer): the
@@ -796,6 +825,9 @@ def main():
             "value": r["samples_per_sec"], "unit": "samples/s", "cores": r["cores"],
             "kind": r["kind"], "host_cores_available": os.cpu_count(),
             "sample": cpu_sample_text(r, B)}
+    if dumped is not None:
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

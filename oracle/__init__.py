@@ -15,11 +15,13 @@ Contents
                     by bench.py as the timed "reference CPU path" (kind=port)
   gen_golden.py     imports the REAL reference (with gym_shim/) in the build
                     container and writes tests/golden/*.npz
-  refimport.py      helper that puts /root/reference + gym_shim on sys.path
+  gen_golden_differential.py  the reference's side of the randomised
+                    differential tests, as tests/golden/ref_*.npz
+  digest.py         bit-exact fixture arrays stored by SHA-256 when large
+  refimport.py      helper that puts the reference tree + gym_shim on sys.path
 
 Parity status: pinned.  Every restatement here is checked against fixtures
-generated from the real reference (tests/golden/, script committed) and,
-when /root/reference is present, live against the imported reference.
+generated from the real reference (tests/golden/, scripts committed).
 """
 import ctypes
 import os

@@ -364,12 +364,14 @@ def gen_seeded_init():
 
     import pfrl
 
+    from oracle.digest import store_exact
+
     g = {}
 
     def rec(name, make):
         torch.manual_seed(11)
         for k, v in make().state_dict().items():
-            g[name + "__" + k] = v.numpy().copy()
+            store_exact(g, name + "__" + k, v.numpy())
 
     def noisy():
         q = pfrl.q_functions.DistributionalFCStateQFunctionWithDiscreteAction(

@@ -1,9 +1,9 @@
-"""Import the REAL reference (pfnet/pfrl) in the build container.
+"""Import the REAL reference (pfnet/pfrl).
 
-TEST INFRASTRUCTURE ONLY.  /root/reference is read-only and does not exist on
-the GPU box, so this is used only by oracle/gen_golden.py and by the
-``-m "not gpu"`` tests that re-validate the oracle live (skipped when the
-reference is absent).
+TEST INFRASTRUCTURE ONLY.  The reference tree (PFRL_REFERENCE_ROOT) is read-only
+and only present where fixtures are generated, so this is used by the
+oracle/gen_golden*.py generators and by bench.py's CPU baseline, never by the
+tests: they compare against what the generators recorded under tests/golden/.
 """
 import os
 import sys

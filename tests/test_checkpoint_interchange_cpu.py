@@ -80,6 +80,7 @@ def test_same_torch_seed_gives_the_reference_initial_weights():
     (tests/golden/ref_seeded_init.npz, oracle/gen_golden.py:gen_seeded_init), so a
     script that only sets the seed starts from the same network."""
     import pfrl_b200 as lib
+    from oracle.digest import assert_exact
 
     g = np.load(os.path.join(GOLD, "ref_seeded_init.npz"))
 
@@ -99,4 +100,4 @@ def test_same_torch_seed_gives_the_reference_initial_weights():
     for name, make in makers.items():
         torch.manual_seed(11)
         for k, v in make().state_dict().items():
-            np.testing.assert_array_equal(v.numpy(), g[name + "__" + k], err_msg=name + "." + k)
+            assert_exact(g, name + "__" + k, v.numpy())

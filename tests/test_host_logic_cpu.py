@@ -137,45 +137,46 @@ def test_vector_frame_stack_shares_frame_objects():
     assert venv.num_envs == 3
 
 
+EXPLORER_CASES = [
+    ("ConstantEpsilonGreedy", (0.3, lambda: np.random.randint(4)), "discrete"),
+    ("LinearDecayEpsilonGreedy", (1.0, 0.1, 20, lambda: np.random.randint(4)), "discrete"),
+    ("ExponentialDecayEpsilonGreedy", (1.0, 0.05, 0.9, lambda: np.random.randint(4)), "discrete"),
+    ("Boltzmann", (0.7,), "discrete"),
+    ("Greedy", (), "discrete"),
+    ("AdditiveGaussian", (0.3, -1, 1), "continuous"),
+    ("AdditiveOU", (0.1, 0.2, 0.4), "continuous"),
+]
+
+
+def _explorer_trace(explorers, av_cls, name):
+    """40 actions of explorer `name` from `explorers` (the reference's module or
+    this package's), the position of numpy's global stream after them, and its repr."""
+    (args, kind), = [(a, k) for n, a, k in EXPLORER_CASES if n == name]
+    q = torch.tensor([[0.3, -0.2, 1.1, 0.4]])
+    ex = getattr(explorers, name)(*args)
+    np.random.seed(5)
+    acts = []
+    for t in range(40):
+        if kind == "discrete":
+            a = ex.select_action(t, lambda: 2, action_value=av_cls(q))
+        else:
+            a = ex.select_action(t, lambda: np.float32([0.2, -0.4]))
+        acts.append(np.asarray(a, dtype=np.float64))
+    return np.stack(acts), np.random.get_state()[1][:8].copy(), repr(ex)
+
+
 def test_explorers_consume_the_reference_stream():
-    """Every explorer against the real reference when it is present (build
-    container): same actions and same position of numpy's global stream."""
-    import pytest
-
-    from oracle import refimport
-
-    if not refimport.available():
-        pytest.skip("reference tree not present")
-    pfrl = refimport.import_reference()
+    """Every explorer against the real reference (tests/golden/ref_explorers.npz,
+    oracle/gen_golden_differential.py): same actions, same position of numpy's
+    global stream and the same repr."""
     from pfrl_b200 import action_value, explorers
 
-    q = torch.tensor([[0.3, -0.2, 1.1, 0.4]])
-    cases = [
-        ("ConstantEpsilonGreedy", (0.3, lambda: np.random.randint(4)), "discrete"),
-        ("LinearDecayEpsilonGreedy", (1.0, 0.1, 20, lambda: np.random.randint(4)), "discrete"),
-        ("ExponentialDecayEpsilonGreedy", (1.0, 0.05, 0.9, lambda: np.random.randint(4)), "discrete"),
-        ("Boltzmann", (0.7,), "discrete"),
-        ("Greedy", (), "discrete"),
-        ("AdditiveGaussian", (0.3, -1, 1), "continuous"),
-        ("AdditiveOU", (0.1, 0.2, 0.4), "continuous"),
-    ]
-    for name, args, kind in cases:
-        outs = []
-        for lib, av_cls in ((pfrl, pfrl.action_value.DiscreteActionValue),
-                            (explorers, action_value.DiscreteActionValue)):
-            ex = getattr(lib.explorers if lib is pfrl else lib, name)(*args)
-            np.random.seed(5)
-            acts = []
-            for t in range(40):
-                if kind == "discrete":
-                    a = ex.select_action(t, lambda: 2, action_value=av_cls(q))
-                else:
-                    a = ex.select_action(t, lambda: np.float32([0.2, -0.4]))
-                acts.append(np.asarray(a, dtype=np.float64))
-            outs.append((np.stack(acts), np.random.get_state()[1][:8].copy(), repr(ex)))
-        np.testing.assert_array_equal(outs[0][0], outs[1][0], err_msg=name)
-        assert np.array_equal(outs[0][1], outs[1][1]), name
-        assert outs[0][2] == outs[1][2], name
+    g = np.load(os.path.join(GOLD, "ref_explorers.npz"))
+    for name, _, _ in EXPLORER_CASES:
+        acts, stream, rep = _explorer_trace(explorers, action_value.DiscreteActionValue, name)
+        np.testing.assert_array_equal(g[name + "_actions"], acts, err_msg=name)
+        assert np.array_equal(g[name + "_stream"], stream), name
+        assert str(g[name + "_repr"]) == rep, name
 
 
 def test_linear_interpolation_hook():
