@@ -154,7 +154,10 @@ __global__ void __launch_bounds__(256) k_ppo_loss(PpoArgs a)
             const float vc = fminf(fmaxf(v, lo), hi);
             const float dc = vc - vt;
             const float lc = dc * dc;
-            const float pass = (v >= lo && v <= hi) ? 1.0f : 0.0f;
+            // d vc / dv of min(max(v, lo), hi) (ppo.py:28-33): autograd gives half the
+            // gradient to each side of a max / min tie, so v == lo or v == hi passes 0.5
+            const float pass = (v > lo ? 1.0f : v == lo ? 0.5f : 0.0f) *
+                               (v < hi ? 1.0f : v == hi ? 0.5f : 0.0f);
             if (lc > lvi) {
                 lvi = lc;
                 gv = 2.0f * dc * pass;

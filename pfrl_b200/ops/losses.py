@@ -1,6 +1,8 @@
 """Fused loss ops (forward + backward CUDA kernels in csrc/losses.cu) as
-torch.autograd Functions.  Inputs must be contiguous fp32 CUDA tensors; there
-is no CPU path here -- agents fall back to their torch formulation on CPU."""
+torch.autograd Functions.  Inputs are CUDA tensors of any float (or bool / integer
+for ``terminal``) dtype and any layout; each is converted to a contiguous fp32 copy
+that stays referenced until the launch has been enqueued.  There is no CPU path
+here -- agents fall back to their torch formulation on CPU."""
 import ctypes
 
 import torch
@@ -28,7 +30,9 @@ class _C51Loss(torch.autograd.Function):
     def forward(ctx, y, next_p, reward, discount, terminal, weights, z, mean):
         L = _lib.load()
         B, n = y.shape
-        yc, pc = _f32(y), _f32(next_p)
+        # every converted input stays bound to a local until the launch: _p keeps only the
+        # address, and a temporary freed early is handed to the next conversion
+        yc, pc, rc, dc, tc = _f32(y), _f32(next_p), _f32(reward), _f32(discount), _f32(terminal)
         w = None if weights is None else _f32(weights)
         zc = _f32(z)
         t = torch.empty_like(yc)
@@ -36,7 +40,7 @@ class _C51Loss(torch.autograd.Function):
         scratch = torch.empty(B, dtype=torch.float32, device=y.device)
         loss = torch.empty((), dtype=torch.float32, device=y.device)
         _lib.check(L.b2rl_c51_loss_fwd(
-            _p(yc), _p(pc), _p(_f32(reward)), _p(_f32(discount)), _p(_f32(terminal)), _p(w),
+            _p(yc), _p(pc), _p(rc), _p(dc), _p(tc), _p(w),
             _p(zc), B, n, int(mean), _p(t), _p(delta), _p(scratch), _p(loss), _stream()))
         ctx.save_for_backward(yc, t, w if w is not None else torch.empty(0, device=y.device))
         ctx.has_w = w is not None
@@ -71,7 +75,8 @@ class _TdLoss(torch.autograd.Function):
     def forward(ctx, q, action, next_q, reward, discount, terminal, weights, clip_delta, mean):
         L = _lib.load()
         B, nA = q.shape
-        qc = _f32(q)
+        # converted inputs stay referenced until the launch (see _C51Loss.forward)
+        qc, nqc, rc, dc, tc = _f32(q), _f32(next_q), _f32(reward), _f32(discount), _f32(terminal)
         act = action.detach().long().contiguous()
         w = None if weights is None else _f32(weights)
         dev = q.device
@@ -81,9 +86,8 @@ class _TdLoss(torch.autograd.Function):
         scratch = torch.empty(B, dtype=torch.float32, device=dev)
         loss = torch.empty((), dtype=torch.float32, device=dev)
         _lib.check(L.b2rl_td_loss_fwd(
-            _p(qc), _p(act), _p(_f32(next_q)), _p(_f32(reward)), _p(_f32(discount)),
-            _p(_f32(terminal)), _p(w), B, nA, int(clip_delta), int(mean), _p(y), _p(t), _p(delta),
-            _p(scratch), _p(loss), _stream()))
+            _p(qc), _p(act), _p(nqc), _p(rc), _p(dc), _p(tc), _p(w), B, nA, int(clip_delta),
+            int(mean), _p(y), _p(t), _p(delta), _p(scratch), _p(loss), _stream()))
         ctx.save_for_backward(y, t, act, w if w is not None else torch.empty(0, device=dev))
         ctx.has_w = w is not None
         ctx.cfg = (B, nA, int(clip_delta), int(mean))

@@ -1,5 +1,7 @@
 """PPO kernels (csrc/ppo.cu) behind torch: GAE over a [T, E] rollout and the
-fused clipped-surrogate loss as an autograd Function."""
+fused clipped-surrogate loss as an autograd Function.  Inputs are CUDA tensors of any
+float dtype and any layout (``cut``/``valid``: bool or integer); each is converted to a
+contiguous fp32 (uint8) copy that stays referenced until the launch has been enqueued."""
 import ctypes
 
 import torch
@@ -23,7 +25,7 @@ def _f32(t):
 
 
 def gae(reward, nonterminal, v, v_next, cut, gamma, lambd, valid=None):
-    """reward/nonterminal/v/v_next: fp32 CUDA [T, E]; cut/valid: uint8 [T, E].
+    """reward/nonterminal/v/v_next: float CUDA [T, E]; cut/valid: bool or uint8 [T, E].
     Returns (adv [T, E], v_teacher [T, E], stats [2] = mean, std)."""
     L = _lib.load()
     T, E = reward.shape
@@ -32,12 +34,15 @@ def gae(reward, nonterminal, v, v_next, cut, gamma, lambd, valid=None):
     vt = torch.zeros((T, E), dtype=torch.float32, device=dev)
     stats = torch.empty(2, dtype=torch.float32, device=dev)
     scratch = torch.empty(((E + 127) // 128) * 3, dtype=torch.float64, device=dev)
+    # every converted input stays bound to a local until the launch: _p keeps only the
+    # address, and a temporary freed early is handed to the next conversion
+    rc, ntc, vc, vnc = _f32(reward), _f32(nonterminal), _f32(v), _f32(v_next)
     cut = cut.to(torch.uint8).contiguous()
     if valid is not None:
         valid = valid.to(torch.uint8).contiguous()
-    _lib.check(L.b2rl_gae(_p(_f32(reward)), _p(_f32(nonterminal)), _p(_f32(v)), _p(_f32(v_next)),
-                          _p(cut), _p(valid), T, E, float(gamma), float(lambd), _p(adv), _p(vt),
-                          _p(scratch), _p(stats), _stream()))
+    _lib.check(L.b2rl_gae(_p(rc), _p(ntc), _p(vc), _p(vnc), _p(cut), _p(valid), T, E,
+                          float(gamma), float(lambd), _p(adv), _p(vt), _p(scratch), _p(stats),
+                          _stream()))
     return adv, vt, stats
 
 
@@ -53,12 +58,12 @@ class _PpoLoss(torch.autograd.Function):
         g_v = torch.empty(M, dtype=torch.float32, device=dev)
         losses = torch.empty(4, dtype=torch.float32, device=dev)
         scratch = torch.empty(((M + 255) // 256) * 3, dtype=torch.float64, device=dev)
+        # converted inputs stay referenced until the launch (see gae)
+        args = [None if x is None else _f32(x).view(-1)
+                for x in (log_prob, entropy, v_pred, log_prob_old, v_pred_old, adv, v_teacher,
+                          adv_stats)]
         _lib.check(L.b2rl_ppo_loss(
-            _p(_f32(log_prob).view(-1)), _p(_f32(entropy).view(-1)), _p(_f32(v_pred).view(-1)),
-            _p(_f32(log_prob_old).view(-1)),
-            _p(None if v_pred_old is None else _f32(v_pred_old).view(-1)),
-            _p(_f32(adv).view(-1)), _p(_f32(v_teacher).view(-1)),
-            _p(None if adv_stats is None else _f32(adv_stats)), M, float(clip_eps),
+            *[_p(x) for x in args], M, float(clip_eps),
             -1.0 if clip_eps_vf is None else float(clip_eps_vf), float(value_coef),
             float(entropy_coef), _p(g_lp), _p(g_en), _p(g_v), _p(scratch), _p(losses),
             _stream()))
